@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """Headline benchmark: decode tokens/s of the TriForce hierarchy at a 128K prompt (BASELINE.json `metric`).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--dump-outputs DIR]
 
 Workload (N = 1, BASELINE.json configs[1]): Llama2-7B-128K shapes (random-init fp16 weights — no checkpoints offline),
 on-chip, prefill = 124928 synthetic tokens, retrieval budget 4096, chunk 8, gamma 6, T = 0.6, top-p 0.9.
@@ -31,6 +31,7 @@ import json
 import os
 import subprocess
 import sys
+import tempfile
 import threading
 import time
 
@@ -39,6 +40,9 @@ sys.path.insert(0, REPO)
 
 METRIC = "decode tokens/sec at 128K prefill (TriForce, Llama2-7B-128K shapes, budget 4096, gamma 6)"
 UNIT = "tokens/s"
+# the line of the last `--impl reference` run on this host, reused as the `cpu_baseline` of a later `ours` run (outside the tree,
+# which may be read-only)
+REFERENCE_LAST = os.path.join(tempfile.gettempdir(), "triforce_b200_reference_last.json")
 
 
 def parse():
@@ -77,7 +81,20 @@ def parse():
     ap.add_argument("--config", default="cfg2", choices=["cfg2", "cfg3", "cfg4", "cfg5"],
                     help="BASELINE.json configs[1..3]: cfg2 = 7B-128K P 124928 B 4096 gamma 6 (default); cfg3 = LWM shapes (plain RoPE), "
                          "P 130048; cfg4 = 7B-128K P 130048 B 12288 gamma 16 (the TP configuration)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write what the last timed step computed to DIR: tokens.npy (the tokens it produced, "
+                         "float64) and target_probs.npy (the target's probabilities at the rows it verified over the full KV, float32). "
+                         "The full-KV attention then keeps its equal key split (TRIFORCE_ATTN_CALIBRATE=0), so the outputs are "
+                         "bit-reproducible from run to run")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and (args.impl != "ours" or args.config == "cfg5"):
+        ap.error("--dump-outputs applies to the TriForce loop of --impl ours (cfg2, cfg3, cfg4)")
+    if args.dump_outputs:
+        # the split calibrated at start-up follows each SM's measured HBM rate, which varies between processes, and with it the
+        # rounding of the attention sums and so the sampled tokens
+        os.environ["TRIFORCE_ATTN_CALIBRATE"] = "0"
     if args.config == "cfg3":
         args.target, args.prefill = "lwm-128K", 130048
     elif args.config == "cfg4":
@@ -278,8 +295,7 @@ def run_reference_arm(args):
                               "attention in place of flash-attn, eager callables in place of CUDA graphs — no CUDA"},
             "tokens_per_step": r["tokens_per_step"], "cpu_baseline": r, "gpu_launches": 0, "wall_seconds": time.time() - t0,
             "e2e": {"value": r["value"], "unit": UNIT, "h2d_bytes_per_step": 0, "d2h_bytes_per_step": 0}}
-    os.makedirs(os.path.join(REPO, "gpurun_out"), exist_ok=True)
-    with open(os.path.join(REPO, "gpurun_out", "reference_last.json"), "w") as f:
+    with open(REFERENCE_LAST, "w") as f:
         json.dump(dict(line, when=time.time(), args=dict(target=args.target, prefill=args.prefill, budget=args.budget, gamma=args.gamma)), f)
     print(json.dumps(line), flush=True)
 
@@ -287,6 +303,17 @@ def run_reference_arm(args):
 # ---------------------------------------------------------------------------------------------------------------------
 # GPU arm
 # ---------------------------------------------------------------------------------------------------------------------
+def dump_outputs(out_dir: str, run, produced: int, loop: str) -> None:
+    """--dump-outputs: the tokens the last timed step handed back to its caller, and the target's probabilities over the vocabulary
+    at the rows that step verified over the full KV (the distribution its tokens were accepted against or resampled from)."""
+    import numpy as np
+    tokens = run.generated[len(run.generated) - produced:]
+    probs = run.loop.full_probs[:run.records[-1][3] + 1] if loop == "device" else run.full_probs
+    os.makedirs(out_dir, exist_ok=True)
+    np.save(os.path.join(out_dir, "tokens.npy"), np.asarray(tokens, dtype=np.float64))
+    np.save(os.path.join(out_dir, "target_probs.npy"), probs.float().cpu().numpy())
+
+
 def run_ours(args):
     import torch
     import torch.distributed as dist
@@ -337,7 +364,10 @@ def run_ours(args):
     draft = LlamaModel(cfg_d, dsd, device=dev, is_draft=True)
     del tsd, dsd
     torch.cuda.empty_cache()
-    cache = FlashSimpleCache(target, P + args.gen_len + 16)
+    # KV slots past the prompt: --gen_len, or more when the steps of one run (warm-up, timed, e2e) could outgrow it by accepting
+    # every draft, so that --steps K runs K steps whatever K is
+    reserve = max(args.gen_len, (args.warmup + 2 * max(args.steps, args.sweep_steps)) * (gamma + 1) + gamma + 2)
+    cache = FlashSimpleCache(target, P + reserve + 16)
     graph_cache = RetrievalCache(target, max_budget=args.budget, prefill=P, gamma=gamma, chunk_size=args.chunk_size)
     draft_cache = StreamingLLMEvictionCache(draft, start_size=16, recent_size=256 - 16 - gamma, gamma=gamma)
     ge = GraphInferenceEngine(target, cache, graph_cache, draft, draft_cache)
@@ -415,12 +445,14 @@ def run_ours(args):
         w0 = time.time()
         e0.record()
         for _ in range(args.steps):
-            run.step()
+            produced = run.step()
         e1.record()
         barrier()
         w1 = time.time()
         if profiling:
             torch.cuda.profiler.stop()
+        if args.dump_outputs and rank == 0:
+            dump_outputs(args.dump_outputs, run, produced, args.loop)
         dev_ms = e0.elapsed_time(e1)
         tokens = run.n - n0
         inner = run.inner_iterations - inner0
@@ -656,9 +688,6 @@ def run_ours(args):
                                     "and bytes per forward are unchanged; the prompt is prefilled again for every alpha; AR is the line's "
                                     "ar_baseline (weight values do not change its speed)"} if sweep else None,
     }
-    os.makedirs(os.path.join(REPO, "gpurun_out"), exist_ok=True)
-    with open(os.path.join(REPO, "gpurun_out", "bench_last.json"), "w") as f:
-        json.dump(line, f)
     if world == 1:
         # free the engine (80 GB) before the reference legs run in child processes
         del run, ge, cache, graph_cache, draft_cache, target, draft, q, o, ws
@@ -684,8 +713,8 @@ def run_ours(args):
             except Exception as e:
                 line["reference_gpu"] = {"unavailable": repr(e)[:300]}
         if not args.no_cpu_baseline:
-            try:  # the driver runs the reference arm first on the same box: reuse its measurement, else take a short sample
-                last = json.load(open(os.path.join(REPO, "gpurun_out", "reference_last.json")))
+            try:  # a `--impl reference` run on this host shortly before: reuse its measurement, else take a short sample
+                last = json.load(open(REFERENCE_LAST))
                 same = last["args"] == dict(target=args.target, prefill=args.prefill, budget=args.budget, gamma=args.gamma)
                 if same and time.time() - last["when"] < 7200 and time.time() - last["when"] < _uptime_seconds():
                     line["cpu_baseline"] = dict(last["cpu_baseline"], reused="measured by `bench.py --impl reference` on this box "

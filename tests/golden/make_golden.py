@@ -1,6 +1,6 @@
 #!/usr/bin/env python
-"""Generates the committed golden fixtures in this directory FROM THE REFERENCE ITSELF (run in the build container,
-where /root/reference exists).  Usage:  python tests/golden/make_golden.py
+"""Generates the committed golden fixtures in this directory FROM THE REFERENCE ITSELF (run where a checkout of the
+reference is at $TRIFORCE_REFERENCE_ROOT, see `oracle/ref_harness.py`).  Usage:  python tests/golden/make_golden.py [which ...]
 
 The reference ships no tests or golden vectors (SURVEY.md §4), so these fixtures — outputs of the reference's own
 Python (`models/cache.py`, `utils/sampling.py`, `utils/decoding.py`, `models/modeling_llama*.py`) executed on CPU under
@@ -13,6 +13,10 @@ Files written:
   forward.npz           reference target forward: last-token logits after a chunked prefill, retrieval-verify logits
   e2e_<cfg>.json        event traces (every sample / rand / Middle_Spec return / target input) of TriForce first and
                         second call (the draft-cache reset quirk, SURVEY §7 hard part 3) and of Autoregressive
+  tree_512.json         the reference's SpecTree rounds over the 512-node tree
+  reference_tree_512.json   the reference's tree/512.pt (roots, branches, Successors, depth; mask rows as packed bits)
+  reference_cli_flags.json  every flag of the reference's test/*.py entry points with its default
+  pg19_sample/, dataset_gs.npz   24 PG-19 books cut to 2000 characters, and the reference's get_dataset('gs') on them
 """
 from __future__ import annotations
 
@@ -241,8 +245,90 @@ def make_tree():
         json.dump(dict(case=case, first_token=first, rounds=rounds), f)
 
 
+def make_reference_tree():
+    """The reference's tree/512.pt, re-encoded as JSON (the 512 x 512 0/1 mask as one packed-bits hex string per row)."""
+    g = torch.load(os.path.join(rh.REF_ROOT, "tree", "512.pt"), weights_only=False)
+    mask = g["mask"].numpy()
+    assert set(np.unique(mask).tolist()) <= {0, 1}
+    out = dict(size=int(g["size"]), roots=g["roots"], branches=g["branches"], Successors=g["Successors"],
+               depth=[int(x) for x in g["depth"].tolist()], mask_rows=[np.packbits(row.astype(np.uint8)).tobytes().hex() for row in mask])
+    with open(os.path.join(HERE, "reference_tree_512.json"), "w") as f:
+        json.dump(out, f)
+
+
+def make_cli_flags():
+    """Every `add_argument('--flag', ...)` of the reference's three entry points: its default as written there, or store_true."""
+    import re
+    out = {}
+    for entry in ("on_chip", "offloading_TP", "offloading_seqouia"):
+        flags = []
+        for flag, rest in re.findall(r"add_argument\('--(\w+)'(.*?)\)\n", open(os.path.join(rh.REF_ROOT, "test", entry + ".py")).read()):
+            m = re.search(r"default=([^,)]+)", rest)
+            flags.append([flag, m.group(1).strip().strip("'").strip('"') if m else None, "store_true" in rest])
+        out[entry] = flags
+    with open(os.path.join(HERE, "reference_cli_flags.json"), "w") as f:
+        json.dump(out, f, indent=1)
+
+
+def make_dataset():
+    """A PG-19 sample (the first 12 books of each of the reference's jsonl files, files in sorted order, every book cut to its
+    first 2000 characters) and the reference's own `get_dataset('gs')` on it with the byte tokenizer of tests/test_dataset_cpu.py.
+    The reference reads the files through `datasets.load_dataset("json", data_files=[...], split="train")`; that package is
+    stood in for by the rows of the given files in order (what the json builder yields for one-object-per-line files)."""
+    import importlib.util
+    import shutil
+    import tempfile
+    import types
+    from test_dataset_cpu import ByteTokenizer
+
+    src = os.path.join(rh.REF_ROOT, "data", "pg19")
+    rows = []
+    for name in sorted(os.listdir(src)):
+        with open(os.path.join(src, name), encoding="utf-8") as f:
+            books = [json.loads(line)["text"] for line in f if line.strip()]
+        rows += [b[:2000] for b in books[:12]]
+    sample_dir = os.path.join(HERE, "pg19_sample")
+    os.makedirs(sample_dir, exist_ok=True)
+    with open(os.path.join(sample_dir, "pg19-sample.json"), "w", encoding="utf-8") as f:
+        for t in rows:
+            f.write(json.dumps({"text": t}) + "\n")
+
+    def load_dataset(kind, data_files, split):
+        assert kind == "json" and split == "train"
+        out = []
+        for p in data_files:
+            with open(p, encoding="utf-8") as f:
+                out += [json.loads(line) for line in f if line.strip()]
+        return out
+
+    shim = types.ModuleType("datasets")
+    shim.load_dataset = load_dataset
+    saved, cwd = sys.modules.get("datasets"), os.getcwd()
+    sys.modules["datasets"] = shim
+    try:
+        spec = importlib.util.spec_from_file_location("ref_dataset", os.path.join(rh.REF_ROOT, "data", "dataset.py"))
+        ref = importlib.util.module_from_spec(spec)
+        spec.loader.exec_module(ref)
+        with tempfile.TemporaryDirectory() as tmp:
+            os.makedirs(os.path.join(tmp, "data", "pg19"))
+            shutil.copy(os.path.join(sample_dir, "pg19-sample.json"), os.path.join(tmp, "data", "pg19"))
+            os.chdir(tmp)  # the reference opens "data/pg19/" relative to the working directory
+            got = ref.get_dataset("gs", tokenizer=ByteTokenizer())
+    finally:
+        os.chdir(cwd)
+        if saved is None:
+            sys.modules.pop("datasets")
+        else:
+            sys.modules["datasets"] = saved
+    assert len(got) == 20 and all(t.dtype == torch.long and t.dim() == 2 and t.shape[0] == 1 for t in got)
+    ids = torch.cat([t[0] for t in got]).numpy()
+    assert ids.min() >= 0 and ids.max() < 2 ** 16
+    np.savez_compressed(os.path.join(HERE, "dataset_gs.npz"), ids=ids.astype(np.uint16),
+                        lengths=np.array([t.shape[1] for t in got], dtype=np.int64))
+
+
 if __name__ == "__main__":
-    which = sys.argv[1:] or ["retrieval", "sampling", "forward", "e2e", "tree"]
+    which = sys.argv[1:] or ["retrieval", "sampling", "forward", "e2e", "tree", "reference_tree", "cli_flags", "dataset"]
     with torch.inference_mode():
         if "retrieval" in which:
             make_retrieval_build()
@@ -254,3 +340,9 @@ if __name__ == "__main__":
             make_e2e()
         if "tree" in which:
             make_tree()
+    if "reference_tree" in which:
+        make_reference_tree()
+    if "cli_flags" in which:
+        make_cli_flags()
+    if "dataset" in which:
+        make_dataset()

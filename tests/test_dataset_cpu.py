@@ -1,9 +1,10 @@
-"""Input pipeline (SURVEY §8 row f-4): `data.dataset.get_dataset` against hand-made jsonl books and — in the build container, where
-the reference checkout and the `datasets` package exist — against the reference's own `get_dataset` on its own PG-19 files."""
+"""Input pipeline (SURVEY §8 row f-4): `data.dataset.get_dataset` against hand-made jsonl books and against what the reference's
+own `get_dataset` returned on a sample of its PG-19 files."""
 import json
 import os
 import sys
 
+import numpy as np
 import pytest
 import torch
 
@@ -61,30 +62,12 @@ def test_lwm_chat_wrapper_truncates_and_wraps():
     assert text.endswith("ASSISTANT: ")
 
 
-_REF_CHILD = r"""
-import importlib.util, os, sys, torch
-sys.path.insert(0, os.path.join(sys.argv[1], "tests"))
-from test_dataset_cpu import ByteTokenizer
-spec = importlib.util.spec_from_file_location("ref_dataset", "/root/reference/data/dataset.py")
-ref = importlib.util.module_from_spec(spec)
-spec.loader.exec_module(ref)
-os.chdir("/root/reference")  # the reference opens "data/pg19/" relative to the working directory
-torch.save(ref.get_dataset("gs", tokenizer=ByteTokenizer()), sys.argv[2])
-"""
-
-
-@pytest.mark.skipif(not os.path.isdir("/root/reference/data/pg19"), reason="reference checkout not on this box")
-def test_against_the_reference_get_dataset(tmp_path):
-    """The reference's own get_dataset('gs') on its own PG-19 files, run in a child process whose HF caches point into tmp_path."""
-    pytest.importorskip("datasets")
-    import subprocess
-    out = tmp_path / "ref_gs.pt"
-    env = dict(os.environ, HF_HOME=str(tmp_path / "hf"), HF_DATASETS_CACHE=str(tmp_path / "hf" / "datasets"), HF_DATASETS_OFFLINE="1")
-    r = subprocess.run([sys.executable, "-c", _REF_CHILD, REPO, str(out)], capture_output=True, text=True, timeout=600, env=env)
-    if r.returncode != 0 or not out.exists():
-        pytest.skip(f"reference get_dataset did not run here: {r.stderr[-300:]}")
-    want = torch.load(out)
-    got = get_dataset("gs", ByteTokenizer(), root="/root/reference/data/pg19")
+def test_against_the_reference_get_dataset(golden_dir):
+    """The reference's own get_dataset('gs') on a sample of its PG-19 files (tests/golden/pg19_sample), as stored by
+    tests/golden/make_golden.py in dataset_gs.npz: the 20 id tensors concatenated, and their lengths."""
+    g = np.load(os.path.join(golden_dir, "dataset_gs.npz"))
+    want = np.split(g["ids"].astype(np.int64), np.cumsum(g["lengths"])[:-1])
+    got = get_dataset("gs", ByteTokenizer(), root=os.path.join(golden_dir, "pg19_sample"))
     assert len(got) == len(want) == 20
     for a, b in zip(got, want):
-        assert torch.equal(a, b)
+        assert torch.equal(a, torch.from_numpy(b)[None])

@@ -1,6 +1,7 @@
 """Host-side logic that needs no GPU: configs, noise sources, drop-in import paths, and the tensor-parallel sharding
 algebra under a real 2-process `gloo` group (the N>1 path of bench.py / test/offloading_TP.py uses the same shard
 function and the same all-reduce seams over NCCL)."""
+import json
 import os
 import subprocess
 import sys
@@ -150,14 +151,13 @@ def test_grow_map_matches_the_reference_tree_file_and_the_oracle_mask_packing():
         assert int(gm["depth"][c]) == int(gm["depth"][p]) + 1
     bits = pack_mask_bits(gm["mask"]).numpy().view(np.uint32)
     np.testing.assert_array_equal(bits, orc.pack_tree_mask(mask))
-    # the JSON is a re-encoding of the reference's tree/512.pt (only checkable where the reference is mounted)
-    ref = "/root/reference/tree/512.pt"
-    if os.path.exists(ref):
-        g = torch.load(ref, weights_only=False)
-        assert g["size"] == gm["size"] and g["roots"] == gm["roots"] and g["branches"] == gm["branches"]
-        assert g["Successors"] == gm["Successors"]
-        assert torch.equal((g["mask"] == 0) if g["mask"].dtype != torch.bool else g["mask"], gm["mask"].bool()) or \
-            torch.equal(g["mask"].bool(), gm["mask"].bool())
+    # the JSON is a re-encoding of the reference's tree/512.pt, whose contents tests/golden/reference_tree_512.json holds
+    g = json.load(open(os.path.join(REPO, "tests", "golden", "reference_tree_512.json")))
+    g["mask"] = torch.from_numpy(np.stack([np.unpackbits(np.frombuffer(bytes.fromhex(r), np.uint8))[:g["size"]] for r in g.pop("mask_rows")]).astype(np.int64))
+    assert g["size"] == gm["size"] and g["roots"] == gm["roots"] and g["branches"] == gm["branches"]
+    assert g["Successors"] == gm["Successors"]
+    assert torch.equal((g["mask"] == 0) if g["mask"].dtype != torch.bool else g["mask"], gm["mask"].bool()) or \
+        torch.equal(g["mask"].bool(), gm["mask"].bool())
 
 
 def test_tree_sampling_tables_match_the_restated_script_helpers():
@@ -198,27 +198,22 @@ def test_tree_noise_is_replayable_and_never_one():
 
 def test_entry_points_keep_the_reference_command_line():
     """test/on_chip.py, test/offloading_TP.py, test/offloading_seqouia.py: every flag of the reference with the reference's
-    default (checked against the reference's own argparse blocks where /root/reference is mounted)."""
-    import re
-
+    default (checked against the flags of the reference's own argparse blocks, stored in tests/golden/reference_cli_flags.json)."""
     from triforce_b200 import cli
 
+    ref_flags = json.load(open(os.path.join(REPO, "tests", "golden", "reference_cli_flags.json")))
     for entry in ("on_chip", "offloading_TP", "offloading_seqouia"):
         ns = vars(cli.build_parser(entry).parse_args([]))
         assert ns["prefill"] in (32768, 130048) and ns["temp"] == 0.6 and ns["top_p"] == 0.9
         script = os.path.join(REPO, "test", entry + ".py")
         out = subprocess.run([sys.executable, script, "--help"], capture_output=True, text=True, timeout=120)
         assert out.returncode == 0 and "--prefill" in out.stdout  # parses its flags without touching CUDA
-        ref = f"/root/reference/test/{entry}.py"
-        if not os.path.exists(ref):
-            continue
-        for flag, rest in re.findall(r"add_argument\('--(\w+)'(.*?)\)\n", open(ref).read()):
+        assert len(ref_flags[entry]) >= 12
+        for flag, want, store_true in ref_flags[entry]:
             assert flag in ns, f"{entry}: flag --{flag} of the reference is missing"
-            m = re.search(r"default=([^,)]+)", rest)
-            if m:
-                want = m.group(1).strip().strip("'").strip('"')
+            if want is not None:
                 assert str(ns[flag]) == want, f"{entry}: --{flag} default {ns[flag]!r} != reference {want!r}"
-            elif "store_true" in rest:
+            elif store_true:
                 assert ns[flag] is False
 
 

@@ -68,7 +68,7 @@ def test_distributed_llama_world1_replays_reference_trace(case):
     _assert_matches_golden(_run(1, case), case)
 
 
-@pytest.mark.skipif(torch.cuda.device_count() < 2, reason="needs two GPUs (run with gpurun --gpus 2)")
+@pytest.mark.skipif(torch.cuda.device_count() < 2, reason="needs two GPUs")
 @pytest.mark.parametrize("case", ["tiny", "g16"])
 def test_distributed_llama_world2_replays_reference_trace(case):
     _assert_matches_golden(_run(2, case), case)
@@ -87,7 +87,7 @@ def test_device_loop_on_the_tp_engine_world1(case, seed):
     _assert_device_loop(1, case, seed)
 
 
-@pytest.mark.skipif(torch.cuda.device_count() < 2, reason="needs two GPUs (run with gpurun --gpus 2)")
+@pytest.mark.skipif(torch.cuda.device_count() < 2, reason="needs two GPUs")
 @pytest.mark.parametrize("case,seed", [("tiny", 3), ("g16", 7)])
 def test_device_loop_on_the_tp_engine_world2(case, seed):
     """... head-sharded over two ranks: the LL seam (projection pushes, add+RMSNorm polls) inside the conditional WHILE graph.  Whether

@@ -205,6 +205,7 @@ class TriForceRun:
         if pad:
             eng.kv_cache.seq_len -= pad  # the padding rows were appended too: roll them back at once
         probs = norm_logits(logits[0], temperature=self.temperature, top_k=self.top_k, top_p=self.top_p)
+        self.full_probs = probs[:len(ids)]  # the target's distribution at the verified rows, kept for inspection
 
         gen_dev = verify_tokens[0, 1:]
         mark = noise.mark()

@@ -115,6 +115,7 @@ class DeviceLoop:
             ops.loop_prepare_full(self.st, self.out_ids, self.first_token, self.full_ids)
             logits = eng.model.forward_target(self.full_ids, kv, None, None, spec=False, use_device_len=True)
             probs = norm_logits(logits[0], temperature=temperature, top_k=-1, top_p=top_p)
+            self.full_probs = probs  # [gamma+2, V]; the captured graph rewrites it on every launch
             ops.loop_verify(probs, self.spec_probs, self.out_ids, self.st, self.rng, strict_less, eos, self.first_token, self.res, self.tokens,
                             self.pass_tokens, kv.seq_len_dev)
             gc.update_graph_cache(kv, use_device_len=True, max_new=max_new)
